@@ -27,6 +27,13 @@ A "step" is one iteration over the whole volume.  `value` = voxels * K / t with 
 iteration driven through the public host-buffer call `CPSolver.step_host_async`: every step uploads the data term x0 from
 pinned host memory, runs the iteration, downloads the current image x and the energy (three steps in flight).  The state
 per GPU (23.6 GB for C4) is far larger than the 126 MB L2, so no L2 flush is needed between iterations.
+
+--dump-outputs DIR writes what the timed path computed in its last timed step as DIR/<name>.npy (one file per rank, suffix
+_rank<r>, when N > 1): C4 / C3 the image x (float32) and the energy (float64); C5 per scheme the tv value (float64) and
+the sub-gradient G, D x and D_T D x (float32).  The float32 arrays of all ranks share 48 MiB; an array larger than its
+share is stored as the elements at fixed seeded flat positions.  The inputs are seeded, so two builds run with the same
+arguments can be compared file by file.  C5 gathers those elements inside its last timed step (the fields of the four
+schemes do not fit in memory together), which adds 12 small gather kernels to the time of a run with --dump-outputs.
 """
 import argparse
 import json
@@ -40,9 +47,11 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the source tree (it may be read-only)
 
 UNIT = "voxel-updates/s"
 LAM = 0.1
+DUMP_BYTES = 48 << 20               # --dump-outputs: bytes of float32 output samples of all ranks (the files stay below 64 MB)
 
 WORKLOADS = {
     # name: slab per GPU, scheme weights, gate sample, CPU-arm sample per process
@@ -179,8 +188,8 @@ def run_reference_arm(args):
         cores = os.cpu_count() or 1
     procs = max(1, min(cores, 64))
     sample = tuple(w["cpu_sample"])
-    # bound the run to a few minutes: one iteration of this sample takes ~2.5 s on one core
-    steps = min(max(1, args.steps), 20)
+    # one iteration of this sample takes ~2.5 s on one core
+    steps = args.steps
     warmup = min(max(0, args.warmup), 3)
     t0 = time.perf_counter()
     with mp.get_context("fork").Pool(procs) as pool:
@@ -433,6 +442,28 @@ def init_dist(dev):
         os.close(saved)
 
 
+# --dump-outputs
+def sample_positions(numel, n, dev):
+    """`n` flat positions in [0, numel) drawn from a fixed seed (the same in every run), or None when all `numel` fit."""
+    import torch
+    if numel <= n:
+        return None
+    return torch.from_numpy(np.random.RandomState(0).randint(0, numel, size=n, dtype=np.int64)).to(dev)
+
+
+def take(t, pos):
+    """The elements of `t` at the flat positions `pos` (all of `t` when None), as a new tensor on t's device."""
+    return t.detach().clone() if pos is None else t.detach().reshape(-1)[pos]
+
+
+def write_outputs(out_dir, arrays, rank, world):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if hasattr(a, "cpu") else a
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ("_rank%d" % rank if world > 1 else "") + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -546,6 +577,9 @@ def run_ours(args):
     t_ms = start.elapsed_time(end)
     clocks = sampler.stop() if sampler else None
     energy = solver.energy()
+    if args.dump_outputs:      # before the end-to-end timing below iterates the solver further
+        pos = sample_positions(solver.x.numel(), DUMP_BYTES // world // 4, dev)
+        write_outputs(args.dump_outputs, {"x": take(solver.x, pos), "energy": np.array([energy], np.float64)}, rank, world)
     dual_ms = sum(e[0].elapsed_time(e[1]) for e in ev) / K
     primal_ms = sum(e[1].elapsed_time(e[2]) for e in ev) / K
     per_rank = None
@@ -709,7 +743,7 @@ def run_c5(args, dev, rank, world, gate, mg_check, barrier):
     Nd_of = {}
     tv_vals = {}
 
-    def one_pass(record):
+    def one_pass(record, dump=None, pos=None):
         for s in SCHEMES:
             e = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
             e[0].record()
@@ -721,6 +755,9 @@ def run_c5(args, dev, rank, world, gate, mg_check, barrier):
             e[3].record()
             Nd_of[s] = int(Dx.shape[1])
             tv_vals[s] = float(tvv)
+            if dump is not None:      # gathered on the device here: the fields of all four schemes do not fit in memory together
+                dump.update({"tv_" + s: np.array([tv_vals[s]], np.float64), "G_" + s: take(G, pos[G.numel()]), "D_" + s: take(Dx, pos[Dx.numel()]),
+                             "D_T_" + s: take(out, pos[out.numel()])})
             del G, Dx, out
             if record:
                 torch.cuda.synchronize()
@@ -736,14 +773,20 @@ def run_c5(args, dev, rank, world, gate, mg_check, barrier):
     launches0 = lib.pytvb_launch_count()
     start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
+    dump, pos = None, None
+    if args.dump_outputs:      # the positions are drawn before the timed region; the last timed step only gathers
+        dump = {}
+        pos = {m: sample_positions(m, DUMP_BYTES // world // 4 // (3 * len(SCHEMES)), dev) for m in [V_local] + [Nd_of[s] * V_local for s in SCHEMES]}
     start.record()
-    for _ in range(K):
-        one_pass(True)
+    for k in range(K):
+        one_pass(True, dump if k == K - 1 else None, pos)
     end.record()
     barrier()
     launches = lib.pytvb_launch_count() - launches0
     clocks = sampler.stop() if sampler else None
     t_ms = start.elapsed_time(end)
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump, rank, world)
     flat = torch.tensor([times[s][o] / K for s in SCHEMES for o in ("tv", "D", "D_T")] + [t_ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(flat, op=dist.ReduceOp.MAX)
@@ -809,7 +852,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true", help="leave the cpu_baseline object out of the line")
     ap.add_argument("--no-parity-gate", action="store_true", help="skip the parity gate and the multi-GPU check (profiling runs under ncu only)")
     ap.add_argument("--no-extras", action="store_true", help="skip the informational reduced-precision measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference_arm(args)
     else:
