@@ -144,6 +144,18 @@ int pytvb_cp_primal_p2p(const pytvb_problem* pb, int variant, const void* y, voi
                         double* d_fid_or_null, const void* halo_lo, const void* halo_hi, void* mirror_prev, void* mirror_next, void* ws,
                         void* stream);
 
+/* Pass B of the ROF-form iteration with another data term: sum_v w_v phi(x_v - x0_v), phi = 0.5 r^2 (L2) or |r| (L1).
+ * With v = x - tau D^T y:   L2: x <- (v + tau w x0) / (1 + tau w)
+ *                           L1: x <- x0 + sign(v - x0) max(|v - x0| - tau w, 0)   (soft threshold)
+ * then xbar <- x_new + theta (x_new - x_old).  Pass A (pytvb_cp_dual) is unchanged.
+ * data_weight: device (Nz, M, Ni, Nj) array of `dtype`, >= 0, or NULL (w = 1).  L2 without a weight map is pytvb_cp_primal_rof.
+ * d_fid_or_null[0] = sum_v w_v (x_new - x0)^2 (L2) or sum_v w_v |x_new - x0| (L1).
+ * mirror_prev / mirror_next: as pytvb_cp_primal_p2p (NULL: no peer push).  halos: as pytvb_DT. */
+typedef enum { PYTVB_DATA_L2 = 0, PYTVB_DATA_L1 = 1 } pytvb_data_term;
+int pytvb_cp_primal_data(const pytvb_problem* pb, int data_term, const void* data_weight, const void* y, void* x, void* xbar,
+                         const void* x0, double tau, double theta, double* d_fid_or_null, const void* halo_lo, const void* halo_hi,
+                         void* mirror_prev, void* mirror_next, void* ws, void* stream);
+
 /* Half-precision STORAGE of the dual field (SURVEY 8f-4): float32 images and arithmetic, y kept as IEEE half in the
  * same (Nz, Nd, M, Ni, Nj) layout, normalised to the unit ball (the array holds y / lam).  Halves the dominant
  * traffic: 4(3Nd+5) -> 6Nd+20 bytes per voxel (68 instead of 116 for Nd = 8).  NOT within the 1e-5 parity

@@ -6,7 +6,9 @@ host.  This module is that loop as a library:
 
   variant="readme"  the README's "simple" iteration, state (x, y_f, y_tv): bit-for-bit the same update order
   variant="rof"     Chambolle & Pock (2011) Alg. 1 for 0.5|x-x0|^2 + lam TV(x), state (x, xbar, y): exact
-                    prox of the data term and over-relaxation
+                    prox of the data term and over-relaxation.  With data_term="l1" and / or a data_weight map w the
+                    data term becomes sum_v w_v |x_v - x0_v| (TV-L1: impulse noise, dead / hot pixels) or
+                    0.5 sum_v w_v (x_v - x0_v)^2 (confidence weights; w = 0 marks missing voxels that TV fills in)
 
 Each iteration is pass A (dual: D(xbar), projection onto the lam-ball, L21 partial sums) and pass B (primal:
 D^T y, data-term update, over-relaxation, fidelity partial sums), i.e. `pytvb_cp_dual` + `pytvb_cp_primal_*`.
@@ -23,6 +25,9 @@ import numpy as np
 import torch
 
 from . import _dev, _lib
+
+
+DATA_TERMS = {"l2": 0, "l1": 1}     # pytvb_data_term
 
 
 def partition_z(Nz_global, world_size):
@@ -71,6 +76,11 @@ class CudaOps:
         fn = self.lib.pytvb_cp_primal_rof if variant == "rof" else self.lib.pytvb_cp_primal_readme
         _lib.check(fn(ctypes.byref(pb), _dev.ptr(y), _dev.ptr(x), _dev.ptr(aux), _dev.ptr(x0), tau, c2, _dev.ptr(d_fid), _dev.ptr(lo), _dev.ptr(hi),
                       _dev.ptr(ws), _dev.stream_ptr()))
+
+    def cp_primal_data(self, pb, data_term, w, y, x, xbar, x0, tau, theta, d_fid, lo, hi, mirror_prev, mirror_next, ws):
+        _lib.check(self.lib.pytvb_cp_primal_data(ctypes.byref(pb), DATA_TERMS[data_term], _dev.ptr(w), _dev.ptr(y), _dev.ptr(x), _dev.ptr(xbar),
+                                                 _dev.ptr(x0), tau, theta, _dev.ptr(d_fid), _dev.ptr(lo), _dev.ptr(hi), mirror_prev, mirror_next,
+                                                 _dev.ptr(ws), _dev.stream_ptr()))
 
     def cp_dual_p2p(self, pb, xbar, y, lam, sigma, d_l21, lo, hi, mirror_prev, mirror_next, ws):
         _lib.check(self.lib.pytvb_cp_dual_p2p(ctypes.byref(pb), _dev.ptr(xbar), _dev.ptr(y), lam, sigma, _dev.ptr(d_l21), _dev.ptr(lo), _dev.ptr(hi),
@@ -217,15 +227,21 @@ class CPSolver:
            separates the passes; "nccl": batched isend/irecv before each pass; "auto" (default, or the environment
            variable PYTVB_COMM): p2p where every rank can set it up, else nccl.  Half-precision duals and injected
            executors always use nccl.
+    data_term : "l2" (default) or "l1": the data term sum_v w_v phi(x_v - x0_v) with phi = 0.5 r^2 or |r|.
+    data_weight : w, broadcast to the slab shape like time_weight (a sharded solver passes its own slab's part), finite and
+                  >= 0; None means w = 1.  w = 0 marks missing data.  With "l2" and no weight the solver is exactly the ROF
+                  solver.  The other data terms need variant="rof" and full-precision duals.
     """
 
     def __init__(self, x0, lam, scheme="hybrid", variant="rof", sigma=0.5, tau=None, theta=1.0, sigma_A=1.0, reg_z_over_reg=1.0,
                  reg_time=0.0, mask_static=False, factor_reg_static=0, distributed=False, group=None, z_offset=None, Nz_global=None,
-                 ops=None, track_energy=True, dual_dtype=None, time_weight=None, comm=None, reduce_group=None):
+                 ops=None, track_energy=True, dual_dtype=None, time_weight=None, comm=None, reduce_group=None, data_term="l2", data_weight=None):
         if scheme not in _dev.SCHEMES:
             raise ValueError("unknown scheme %r" % (scheme,))
         if variant not in ("rof", "readme"):
             raise ValueError("variant must be 'rof' or 'readme'")
+        if data_term not in DATA_TERMS:
+            raise ValueError("data_term must be 'l2' or 'l1'")
         self.ops = ops if ops is not None else CudaOps()
         self.scheme, self.variant = scheme, variant
         self.lam, self.sigma, self.theta, self.sigma_A = float(lam), float(sigma), float(theta), float(sigma_A)
@@ -276,6 +292,22 @@ class CPSolver:
             if self.halo is not None:
                 self.halo.dist.all_reduce(mx, op=self.halo.dist.ReduceOp.MAX, group=self.halo.group)
             max_tw = float(mx.item())
+        # data term: the weight map of this slab, in the image dtype; _w_min = its smallest entry over the whole volume, as stored
+        # (a tiny positive weight may round to 0 in float32, and the dual energy must then be refused)
+        self.data_term = data_term
+        self._dw = None
+        self._w_min = 1.0
+        if data_weight is not None:
+            w = data_weight if isinstance(data_weight, torch.Tensor) else torch.as_tensor(np.asarray(data_weight))
+            w = torch.broadcast_to(w.to(dev).to(torch.float64), shape)
+            if not bool(torch.isfinite(w).all()) or bool((w < 0).any()):
+                raise ValueError("data_weight must be finite and >= 0")
+            self._dw = w.to(dt).contiguous()
+            mn = self._dw.min().double().reshape(1).clone()
+            if self.halo is not None:
+                self.halo.dist.all_reduce(mn, op=self.halo.dist.ReduceOp.MIN, group=self.halo.group)
+            self._w_min = float(mn.item())
+        self._data = data_term != "l2" or self._dw is not None    # pass B through pytvb_cp_primal_data
         self.pb = _lib.make_problem(scheme, _lib.F32 if dt == torch.float32 else _lib.F64, shape, float(reg_z_over_reg), float(reg_time),
                                     float(factor_reg_static), self._ms.data_ptr() if self._ms is not None else None, self.z_offset,
                                     self.Nz_global, self._ts.data_ptr() if self._ts is not None else None)
@@ -299,6 +331,8 @@ class CPSolver:
                 raise ValueError("dual_dtype=torch.float16 needs float32 images and variant='rof'")
             if not self.lam > 0:
                 raise ValueError("half-precision dual storage needs lam > 0")
+        if self._data and (variant != "rof" or self.dual_dtype != dt):
+            raise ValueError("data_term='l1' and data_weight need variant='rof' and full-precision duals")
         self.y = torch.zeros((shape[0], self.Nd) + shape[1:], dtype=self.dual_dtype, device=dev)
         # partial sums of this slab: [0:3] L21(D u) and [3:6] |x - x0|^2, one slot per sub-slab call of a pass
         self.scal = torch.zeros(6, dtype=torch.float64, device=dev)
@@ -411,6 +445,10 @@ class CPSolver:
         lo = self.y[a - 1, self._zf] if a > 0 else self._fld_lo
         hi = self.y[b, self._zb] if b < Nz else self._fld_hi
         d = self.scal[3 + slot:4 + slot] if self.track_energy else None
+        if self._data:
+            self.ops.cp_primal_data(self._sub_problem(a, b), self.data_term, self._dw[a:b] if self._dw is not None else None, self.y[a:b], self.x[a:b],
+                                    self.aux[a:b], self.x0[a:b], self.tau, self.theta, d, lo, hi, None, None, self.ws)
+            return
         c2 = self.theta if self.variant == "rof" else self.sigma_A
         if self.y.dtype == torch.float16:
             self.ops.cp_primal(self.variant, self._sub_problem(a, b), self.y[a:b], self.x[a:b], self.aux[a:b], self.x0[a:b], self.tau, c2, d, lo, hi,
@@ -471,9 +509,13 @@ class CPSolver:
             self.scal[3:6].zero_()
         if self._peer is not None:
             d = self.scal[3:4] if self.track_energy else None
-            c2 = self.theta if self.variant == "rof" else self.sigma_A
-            self.ops.cp_primal_p2p(self.variant, self.pb, self.y, self.x, self.aux, self.x0, self.tau, c2, d, self._fld_lo, self._fld_hi,
-                                   self._mir_B[0], self._mir_B[1], self.ws)
+            if self._data:
+                self.ops.cp_primal_data(self.pb, self.data_term, self._dw, self.y, self.x, self.aux, self.x0, self.tau, self.theta, d, self._fld_lo,
+                                        self._fld_hi, self._mir_B[0], self._mir_B[1], self.ws)
+            else:
+                c2 = self.theta if self.variant == "rof" else self.sigma_A
+                self.ops.cp_primal_p2p(self.variant, self.pb, self.y, self.x, self.aux, self.x0, self.tau, c2, d, self._fld_lo, self._fld_hi,
+                                       self._mir_B[0], self._mir_B[1], self.ws)
             self._peer.barrier()
             self._pending = ()
             return
@@ -513,7 +555,8 @@ class CPSolver:
 
     def _graph_state_key(self):
         """What a captured graph has baked in: buffer addresses and the scalar parameters of the passes."""
-        return (self.x0.data_ptr(), self.x.data_ptr(), self.aux.data_ptr(), self.y.data_ptr(), self.lam, self.sigma, self.tau, self.theta, self.sigma_A)
+        return (self.x0.data_ptr(), self.x.data_ptr(), self.aux.data_ptr(), self.y.data_ptr(), self.lam, self.sigma, self.tau, self.theta, self.sigma_A,
+                self._dw.data_ptr() if self._dw is not None else 0)
 
     def step(self, n=1):
         """Run n iterations; returns self."""
@@ -616,8 +659,11 @@ class CPSolver:
         if self.halo is not None:
             s = s.to(self.x0.device)
             self.halo.allreduce_sum(s)
-        l21, fid = s.tolist()
-        return 0.5 * fid + self.lam * l21
+        return self._energy_of(*s.tolist())
+
+    def _energy_of(self, l21, fid):
+        """Energy from the partial sums of the passes: fid = sum w r^2 (l2) or sum w |r| (l1), r = x - x0."""
+        return (0.5 * fid if self.data_term == "l2" else fid) + self.lam * l21
 
     def energy_async(self):
         """Start the all-reduce of this iteration's energy terms without putting it on the critical path; returns a
@@ -632,19 +678,18 @@ class CPSolver:
         s, work = handle
         if work is not None:
             work.wait()
-        l21, fid = s.tolist()
-        return 0.5 * fid + self.lam * l21
+        return self._energy_of(*s.tolist())
 
     def energy(self):
         """0.5 |x - x0|^2 + lam L21(D u) of the last iteration over the WHOLE volume (u = the image the dual pass
-        differentiated: README.md:157).  One all-reduce of two doubles when sharded; synchronises."""
+        differentiated: README.md:157), with the chosen data term in place of 0.5 |x - x0|^2.  One all-reduce of two doubles
+        when sharded; synchronises."""
         if not self.track_energy:
             raise RuntimeError("energy tracking was disabled")
         s = torch.stack((self.scal[0:3].sum(), self.scal[3:6].sum()))
         if self.halo is not None:
             self.halo.allreduce_sum(s)
-        l21, fid = s.tolist()
-        return 0.5 * fid + self.lam * l21
+        return self._energy_of(*s.tolist())
 
     # ---- primal-dual gap, stopping rule, data-term hook (SURVEY 8f items 1-2) ----------------------------
     def _sync_halos_for_diagnostics(self):
@@ -654,7 +699,8 @@ class CPSolver:
             self._pending = None
 
     def primal_energy(self):
-        """P(x) = 0.5 |x - x0|^2 + lam TV(x) at the current iterate, over the whole volume (synchronises)."""
+        """P(x) = 0.5 |x - x0|^2 + lam TV(x) (or the chosen data term + lam TV(x)) at the current iterate, over the whole volume
+        (synchronises)."""
         lo = hi = None
         if self.halo is not None and self.z_on:
             self._sync_halos_for_diagnostics()
@@ -664,15 +710,26 @@ class CPSolver:
             lo, hi = self._img_lo, self._img_hi
         d = torch.zeros(2, dtype=torch.float64, device=self.x.device)
         self.ops.tv_value(self.pb, self.x, d[0:1], lo, hi, self.ws)
-        d[1] = torch.sum((self.x - self.x0).double() ** 2) if self.x.numel() < (1 << 28) else sum(
-            torch.sum((self.x[k] - self.x0[k]).double() ** 2) for k in range(self.shape[0]))
+        if not self._data:
+            d[1] = torch.sum((self.x - self.x0).double() ** 2) if self.x.numel() < (1 << 28) else sum(
+                torch.sum((self.x[k] - self.x0[k]).double() ** 2) for k in range(self.shape[0]))
+        else:
+            for k in range(self.shape[0]):      # plane by plane: no volume-sized float64 temporaries
+                r = (self.x[k] - self.x0[k]).double()
+                r = r * r if self.data_term == "l2" else r.abs()
+                d[1] += torch.sum(r * self._dw[k].double() if self._dw is not None else r)
         if self.halo is not None:
             self.halo.allreduce_sum(d)
         tv, fid = d.tolist()
-        return 0.5 * fid + self.lam * tv
+        return self._energy_of(tv, fid)
 
     def dual_energy(self):
-        """D(y) = 0.5 |x0|^2 - 0.5 |x0 - D^T y|^2 for the feasible dual iterate y (|y_v|_2 <= lam after the projection)."""
+        """D(y) = 0.5 |x0|^2 - 0.5 |x0 - D^T y|^2 for the feasible dual iterate y (|y_v|_2 <= lam after the projection).
+        Other data terms, with s = D^T y:  weighted l2: sum_v (s x0 - s^2 / (2 w));  l1: c <s, x0> with c = min(1, min_v w_v / |s_v|),
+        the dual scaled into the feasible set |s_v| <= w_v of the conjugate of the data term (a lower bound of the optimum that
+        tends to it).  Where some w_v = 0 the dual objective is unbounded: raises ValueError (solve() then stops on the energy)."""
+        if self._data and not self._w_min > 0:
+            raise ValueError("the dual energy is unbounded where data_weight = 0: no duality gap (solve() uses the energy change)")
         lo = hi = None
         if self.halo is not None and self.z_on:
             to_prev = self.y[0, self._zb] if self.scheme != "upwind" else None
@@ -683,6 +740,8 @@ class CPSolver:
         if self.y.dtype != self.x.dtype:
             raise NotImplementedError("the duality gap is not available with half-precision dual storage")
         self.ops.adjoint(self.pb, self.y, dty, lo, hi)
+        if self._data:
+            return self._dual_energy_data(dty)
         d = torch.zeros(2, dtype=torch.float64, device=self.x.device)
         for k in range(self.shape[0]):          # plane by plane: no volume-sized float64 temporaries
             x0k = self.x0[k].double()
@@ -693,16 +752,39 @@ class CPSolver:
         a, b = d.tolist()
         return 0.5 * a - 0.5 * b
 
+    def _dual_energy_data(self, dty):
+        d = torch.zeros(2, dtype=torch.float64, device=self.x.device)    # l2: [sum, -]; l1: [<s, x0>, max |s| / w]
+        for k in range(self.shape[0]):
+            s, x0k = dty[k].double(), self.x0[k].double()
+            w = self._dw[k].double() if self._dw is not None else None
+            if self.data_term == "l2":
+                d[0] += torch.sum(s * x0k - s * s / (2.0 * w))
+            else:
+                d[0] += torch.sum(s * x0k)
+                d[1] = torch.maximum(d[1], (s.abs() / w if w is not None else s.abs()).max())
+        if self.halo is not None:
+            self.halo.allreduce_sum(d[0:1])
+            self.halo.dist.all_reduce(d[1:2], op=self.halo.dist.ReduceOp.MAX, group=self.halo.group)
+        a, m = d.tolist()
+        if self.data_term == "l2":
+            return a
+        return a * (1.0 / m if m > 1.0 else 1.0)
+
     def gap(self):
-        """(primal, dual, primal - dual); the gap is >= 0 and vanishes at the solution of the ROF problem."""
+        """(primal, dual, primal - dual); the gap is >= 0 and vanishes at the solution.  Raises ValueError when the data weight
+        has zeros (see dual_energy)."""
         p, d = self.primal_energy(), self.dual_energy()
         return p, d, p - d
 
     def solve(self, max_iter=1000, tol=1e-4, check_every=25, callback=None):
         """Iterate until the relative primal-dual gap (P - D) / max(|P|, tiny) <= tol or max_iter is reached.
+        Where the data weight has zeros there is no gap (see dual_energy): the run then stops when the primal energy changes by
+        at most tol relative to its value between two checks, and `D` is None.  info["criterion"] says which rule was used.
         Returns a dict with the number of iterations and the final energies.  `callback(solver, it, P, D)` is called
         at every check (e.g. to record a convergence curve)."""
-        info = dict(iterations=0, converged=False)
+        if self._data and not self._w_min > 0:
+            return self._solve_by_energy(max_iter, tol, check_every, callback)
+        info = dict(iterations=0, converged=False, criterion="gap")
         it = 0
         while it < max_iter:
             n = min(check_every, max_iter - it)
@@ -715,6 +797,25 @@ class CPSolver:
             if g <= tol * max(abs(p), 1e-300):
                 info["converged"] = True
                 break
+        return info
+
+    def _solve_by_energy(self, max_iter, tol, check_every, callback):
+        info = dict(iterations=0, converged=False, criterion="energy")
+        it, p_prev = 0, None
+        while it < max_iter:
+            n = min(check_every, max_iter - it)
+            self.step(n)
+            it += n
+            p = self.primal_energy()
+            if callback is not None:
+                callback(self, it, p, None)
+            info.update(iterations=it, primal=p)
+            if p_prev is not None:
+                info["relative_change"] = abs(p - p_prev) / max(abs(p), 1e-300)
+                if info["relative_change"] <= tol:
+                    info["converged"] = True
+                    break
+            p_prev = p
         return info
 
     def set_data(self, x0, reset_primal=False, reset_dual=False):
@@ -846,7 +947,8 @@ def gd_denoise(x0, lam, n_iter, step, scheme="hybrid", return_pytorch_tensor=Fal
 
 
 def cp_denoise(x0, lam, n_iter, scheme="hybrid", variant="rof", return_pytorch_tensor=False, return_energy=False, **kw):
-    """Denoise `x0` with n_iter fused Chambolle-Pock iterations; see CPSolver for the keyword arguments."""
+    """Denoise `x0` with n_iter fused Chambolle-Pock iterations; see CPSolver for the keyword arguments (e.g. data_term="l1" for
+    impulse noise, data_weight for per-voxel confidence or missing data)."""
     solver = CPSolver(x0, lam, scheme=scheme, variant=variant, track_energy=return_energy, **kw)
     solver.step(int(n_iter))
     if isinstance(x0, torch.Tensor):

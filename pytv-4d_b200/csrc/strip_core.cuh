@@ -479,9 +479,15 @@ PYTVB_HD void strip_quad_DT(T* out, const PrimalPlane<T, YT>& pl, const Params<T
 // Primal update at one quad.  VARIANT 0: ROF prox + over-relaxation (aux = xbar); 1: README form (aux = y_f).
 // c1 = 1/(1+tau) (rof) or 1/(1+sigma_A) (readme); c2 = theta or sigma_A.  Returns sum (x_new - x0)^2.
 // `tau` multiplies D^T y: for a normalised half-precision dual the caller passes tau * lam.
-template <typename T, int VEC, int SCHEME, bool Z_ON, bool T_ON, int VARIANT, bool CG = false, typename YT = T, bool TS = false, bool MIR = false>
+// Other data terms, with v = x - tau D^T y, w = data weight at the voxel (wgt[...] if WM, else 1) and tau_x0 the step of
+// the data term (aux = xbar, c2 = theta, c1 unused):
+//   VARIANT 2: weighted L2, x_new = (v + tau w x0) / (1 + tau w);                  returns sum w (x_new - x0)^2
+//   VARIANT 3: L1,          x_new = x0 + sign(v - x0) max(|v - x0| - tau w, 0);    returns sum w |x_new - x0|
+// (WM is a template parameter for the reason given at strip_raw_diffs_impl.)
+template <typename T, int VEC, int SCHEME, bool Z_ON, bool T_ON, int VARIANT, bool CG = false, typename YT = T, bool TS = false, bool MIR = false,
+          bool WM = false>
 PYTVB_HD T strip_quad_cp_primal(T* x, T* aux, const T* x0, const PrimalPlane<T, YT>& pl, const Params<T>& P, int i, int j0, int o, int o_up, int o_dn,
-                                T tau, T c1, T c2, T tau_x0 = T(-1), MirrorPlanes<T> mir = MirrorPlanes<T>{nullptr, nullptr}) {
+                                T tau, T c1, T c2, T tau_x0 = T(-1), MirrorPlanes<T> mir = MirrorPlanes<T>{nullptr, nullptr}, const T* wgt = nullptr) {
     T dty[VEC];
     strip_quad_DT<T, VEC, SCHEME, Z_ON, T_ON, CG, YT, TS>(dty, pl, P, i, j0, o, o_up, o_dn);
     if (tau_x0 < T(0)) tau_x0 = tau;
@@ -489,7 +495,7 @@ PYTVB_HD T strip_quad_cp_primal(T* x, T* aux, const T* x0, const PrimalPlane<T, 
     const Pack<T, VEC> xo = ld_pack<T, VEC>(x + off), x0q = ld_pack<T, VEC>(x0 + off);
     Pack<T, VEC> xn, ax;
     T fid = T(0);
-    if (VARIANT == 0) {
+    if constexpr (VARIANT == 0) {
 #pragma unroll
         for (int e = 0; e < VEC; ++e) {
             xn.v[e] = (xo.v[e] - tau * dty[e] + tau_x0 * x0q.v[e]) * c1;
@@ -497,7 +503,7 @@ PYTVB_HD T strip_quad_cp_primal(T* x, T* aux, const T* x0, const PrimalPlane<T, 
             const T r = xn.v[e] - x0q.v[e];
             fid += r * r;
         }
-    } else {
+    } else if constexpr (VARIANT == 1) {
         const Pack<T, VEC> yf = ld_pack<T, VEC>(aux + off);
 #pragma unroll
         for (int e = 0; e < VEC; ++e) {
@@ -506,12 +512,36 @@ PYTVB_HD T strip_quad_cp_primal(T* x, T* aux, const T* x0, const PrimalPlane<T, 
             const T r = xn.v[e] - x0q.v[e];
             fid += r * r;
         }
+    } else {
+        static_assert(VARIANT == 2 || VARIANT == 3, "unknown primal variant");
+        Pack<T, VEC> wq;
+        if constexpr (WM) wq = ld_pack<T, VEC>(wgt + off);
+#pragma unroll
+        for (int e = 0; e < VEC; ++e) {
+            T w = T(1), tw = tau_x0;
+            if constexpr (WM) { w = wq.v[e]; tw = tau_x0 * w; }
+            const T v = xo.v[e] - tau * dty[e];
+            T r;
+            if constexpr (VARIANT == 2) {
+                xn.v[e] = (v + tw * x0q.v[e]) / (T(1) + tw);
+                r = xn.v[e] - x0q.v[e];
+                fid += w * (r * r);
+            } else {
+                const T d = v - x0q.v[e];
+                const T a = (d < T(0) ? -d : d) - tw;
+                const T s = a > T(0) ? a : T(0);
+                xn.v[e] = x0q.v[e] + (d < T(0) ? -s : s);
+                r = xn.v[e] - x0q.v[e];
+                fid += w * (r < T(0) ? -r : r);
+            }
+            ax.v[e] = xn.v[e] + c2 * (xn.v[e] - xo.v[e]);
+        }
     }
     st_pack<T, VEC>(x + off, xn);
     st_pack<T, VEC>(aux + off, ax);
     if constexpr (MIR && Z_ON) {
-        // the image the neighbours' next dual pass differentiates: xbar (rof) or x (readme)
-        const Pack<T, VEC>& u = (VARIANT == 0) ? ax : xn;
+        // the image the neighbours' next dual pass differentiates: x (readme) or xbar (every other variant)
+        const Pack<T, VEC>& u = (VARIANT == 1) ? xn : ax;
         if (mir.prev) st_pack<T, VEC>(mir.prev + o, u);
         if (mir.next) st_pack<T, VEC>(mir.next + o, u);
     }
