@@ -156,6 +156,22 @@ int pytvb_cp_primal_data(const pytvb_problem* pb, int data_term, const void* dat
                          const void* x0, double tau, double theta, double* d_fid_or_null, const void* halo_lo, const void* halo_hi,
                          void* mirror_prev, void* mirror_next, void* ws, void* stream);
 
+/* The same iteration with the adjoint split between the passes: fewer bytes per voxel, results bitwise equal to
+ * pytvb_cp_dual followed by pytvb_cp_primal_rof (data_term L2, no weight) or pytvb_cp_primal_data.  M <= 8.
+ * q: device (Nz, M, Ni, Nj) array of `dtype`, scratch written by the dual pass and read by the primal pass of the same
+ * iteration (the in-plane and time part of D^T y).  Other arguments: as pytvb_cp_dual_p2p, and as pytvb_cp_primal_data for
+ * the primal pass; halos and mirrors keep their meaning.  The non-_p2p forms push nothing. */
+int pytvb_cp_dual_adj(const pytvb_problem* pb, const void* xbar, void* y, void* q, double lam, double sigma, double* d_l21_or_null,
+                      const void* halo_lo, const void* halo_hi, void* ws, void* stream);
+int pytvb_cp_dual_adj_p2p(const pytvb_problem* pb, const void* xbar, void* y, void* q, double lam, double sigma, double* d_l21_or_null,
+                          const void* halo_lo, const void* halo_hi, void* mirror_prev, void* mirror_next, void* ws, void* stream);
+int pytvb_cp_primal_adj(const pytvb_problem* pb, int data_term, const void* data_weight, const void* y, const void* q, void* x, void* xbar,
+                        const void* x0, double tau, double theta, double* d_fid_or_null, const void* halo_lo, const void* halo_hi, void* ws,
+                        void* stream);
+int pytvb_cp_primal_adj_p2p(const pytvb_problem* pb, int data_term, const void* data_weight, const void* y, const void* q, void* x, void* xbar,
+                            const void* x0, double tau, double theta, double* d_fid_or_null, const void* halo_lo, const void* halo_hi,
+                            void* mirror_prev, void* mirror_next, void* ws, void* stream);
+
 /* Half-precision STORAGE of the dual field (SURVEY 8f-4): float32 images and arithmetic, y kept as IEEE half in the
  * same (Nz, Nd, M, Ni, Nj) layout, normalised to the unit ball (the array holds y / lam).  Halves the dominant
  * traffic: 4(3Nd+5) -> 6Nd+20 bytes per voxel (68 instead of 116 for Nd = 8).  NOT within the 1e-5 parity

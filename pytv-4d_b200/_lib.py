@@ -69,6 +69,12 @@ _PROTOTYPES = {
     "pytvb_cp_primal_p2p": (ctypes.c_int, [_PB, ctypes.c_int, _VP, _VP, _VP, _VP, ctypes.c_double, ctypes.c_double, _VP, _VP, _VP, _VP, _VP, _VP, _VP]),
     "pytvb_cp_primal_data": (ctypes.c_int, [_PB, ctypes.c_int, _VP, _VP, _VP, _VP, _VP, ctypes.c_double, ctypes.c_double, _VP, _VP, _VP, _VP, _VP, _VP,
                                             _VP]),
+    "pytvb_cp_dual_adj": (ctypes.c_int, [_PB, _VP, _VP, _VP, ctypes.c_double, ctypes.c_double, _VP, _VP, _VP, _VP, _VP]),
+    "pytvb_cp_dual_adj_p2p": (ctypes.c_int, [_PB, _VP, _VP, _VP, ctypes.c_double, ctypes.c_double, _VP, _VP, _VP, _VP, _VP, _VP, _VP]),
+    "pytvb_cp_primal_adj": (ctypes.c_int, [_PB, ctypes.c_int, _VP, _VP, _VP, _VP, _VP, _VP, ctypes.c_double, ctypes.c_double, _VP, _VP, _VP, _VP,
+                                           _VP]),
+    "pytvb_cp_primal_adj_p2p": (ctypes.c_int, [_PB, ctypes.c_int, _VP, _VP, _VP, _VP, _VP, _VP, ctypes.c_double, ctypes.c_double, _VP, _VP, _VP,
+                                               _VP, _VP, _VP, _VP]),
     "pytvb_cp_dual_f16y": (ctypes.c_int, [_PB, _VP, _VP, ctypes.c_double, ctypes.c_double, _VP, _VP, _VP, _VP, _VP]),
     "pytvb_cp_primal_rof_f16y": (ctypes.c_int, [_PB, _VP, _VP, _VP, _VP, ctypes.c_double, ctypes.c_double, ctypes.c_double, _VP, _VP, _VP, _VP, _VP]),
     "pytvb_tv_host": (ctypes.c_int, [_PB, _VP, _VP, _VP, ctypes.POINTER(ctypes.c_double)]),

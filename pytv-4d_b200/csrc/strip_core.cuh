@@ -203,12 +203,13 @@ PYTVB_HD MirrorPlanes<YT> mirror_planes(const MirrorBufs<YT>& m, const PT& P, in
     r.next = (m.next && z == P.Nz - 1) ? m.next + (long long)t * P.sT : nullptr;
     return r;
 }
-template <typename T, int VEC, int SCHEME, bool Z_ON, bool T_ON, typename YT = T, bool TS = false, bool MIR = false>
-PYTVB_HD T strip_quad_cp_dual(const DualPlane<T, YT>& pl, const Params<T>& P, int i, int j0, int o, int o_up, int o_dn, T sig, T lam,
-                              MirrorPlanes<YT> mir = MirrorPlanes<YT>{nullptr, nullptr}) {
+// strip_quad_cp_dual that also leaves the new y of the quad in `y` (the dual pass that finishes part of the adjoint).
+template <typename T, int VEC, int SCHEME, bool Z_ON, bool T_ON, typename YT, bool TS, bool MIR>
+PYTVB_HD T strip_quad_cp_dual_y(T (*y)[VEC], const DualPlane<T, YT>& pl, const Params<T>& P, int i, int j0, int o, int o_up, int o_dn, T sig, T lam,
+                                MirrorPlanes<YT> mir) {
     typedef Comp<SCHEME, Z_ON, T_ON> C;
     constexpr int ND = C::ND;
-    T y[ND][VEC], d[ND][VEC];
+    T d[ND][VEC];
 #pragma unroll
     for (int k = 0; k < ND; ++k) ld_y<T, YT, VEC>(y[k], pl.y + (long long)k * P.sC + o);
     strip_raw_diffs<T, VEC, SCHEME, Z_ON, T_ON, YT, TS>(d, pl, P, i, j0, o, o_up, o_dn);
@@ -230,7 +231,6 @@ PYTVB_HD T strip_quad_cp_dual(const DualPlane<T, YT>& pl, const Params<T>& P, in
         for (int k = 0; k < ND; ++k) y[k][e] *= scale;
     }
 #pragma unroll
-#pragma unroll
     for (int k = 0; k < ND; ++k) st_y<T, YT, VEC>(pl.y + (long long)k * P.sC + o, y[k]);
     if constexpr (MIR && Z_ON) {
         // the previous rank's adjoint reads my backward-type z slot of my first plane, the next rank's my forward-type
@@ -239,6 +239,12 @@ PYTVB_HD T strip_quad_cp_dual(const DualPlane<T, YT>& pl, const Params<T>& P, in
         if (mir.next) st_y<T, YT, VEC>(mir.next + o, y[C::Z_F]);
     }
     return l21;
+}
+template <typename T, int VEC, int SCHEME, bool Z_ON, bool T_ON, typename YT = T, bool TS = false, bool MIR = false>
+PYTVB_HD T strip_quad_cp_dual(const DualPlane<T, YT>& pl, const Params<T>& P, int i, int j0, int o, int o_up, int o_dn, T sig, T lam,
+                              MirrorPlanes<YT> mir = MirrorPlanes<YT>{nullptr, nullptr}) {
+    T y[Comp<SCHEME, Z_ON, T_ON>::ND][VEC];
+    return strip_quad_cp_dual_y<T, VEC, SCHEME, Z_ON, T_ON, YT, TS, MIR>(y, pl, P, i, j0, o, o_up, o_dn, sig, lam, mir);
 }
 
 // D_scheme at one quad, stored to the field plane `out` (component 0 of plane (z,t); component k at + k*sC).
@@ -343,14 +349,102 @@ PYTVB_HD PrimalPlane<T, YT> make_primal_plane(const FieldView<YT>& Y, const Para
     return p;
 }
 
-// minus-side and plus-side operands of one axis given the slot values at k-1 / k / k+1:
+// Arithmetic of the adjoint with its rounding pinned: no contraction into fma.  D^T y is computed in two places - whole in
+// the primal pass, or split into an in-plane / time prefix (dual pass, cp_dual_adj_kernel) and the z term (primal pass) -
+// and both must round identically.
+PYTVB_HD float add_rn(float a, float b) {
+#if defined(__CUDA_ARCH__)
+    return __fadd_rn(a, b);
+#else
+    return a + b;
+#endif
+}
+PYTVB_HD float sub_rn(float a, float b) {
+#if defined(__CUDA_ARCH__)
+    return __fsub_rn(a, b);
+#else
+    return a - b;
+#endif
+}
+PYTVB_HD float mul_rn(float a, float b) {
+#if defined(__CUDA_ARCH__)
+    return __fmul_rn(a, b);
+#else
+    return a * b;
+#endif
+}
+PYTVB_HD double add_rn(double a, double b) {
+#if defined(__CUDA_ARCH__)
+    return __dadd_rn(a, b);
+#else
+    return a + b;
+#endif
+}
+PYTVB_HD double sub_rn(double a, double b) {
+#if defined(__CUDA_ARCH__)
+    return __dsub_rn(a, b);
+#else
+    return a - b;
+#endif
+}
+PYTVB_HD double mul_rn(double a, double b) {
+#if defined(__CUDA_ARCH__)
+    return __dmul_rn(a, b);
+#else
+    return a * b;
+#endif
+}
+
+// One axis term of the adjoint, a * m - b * p, from the slot values at k-1 / k / k+1.  m and p:
 //   upwind: (F[k-1], F[k])   downwind: (B[k], B[k+1])   hybrid: (F[k-1]+B[k], F[k]+B[k+1])   central: (C[k-1], C[k+1])
 template <typename T, int SCHEME>
-PYTVB_HD void adj_operands(T& m, T& p, T f_m, T f_c, T b_c, T b_p, bool fallback) {
+PYTVB_HD T adj_term(T a, T b, T f_m, T f_c, T b_c, T b_p, bool fallback) {
+    T m, p;
     if (SCHEME == UPWIND || (SCHEME == CENTRAL && fallback)) { m = f_m; p = f_c; }
     else if (SCHEME == DOWNWIND) { m = b_c; p = b_p; }
-    else if (SCHEME == HYBRID) { m = f_m + b_c; p = f_c + b_p; }
+    else if (SCHEME == HYBRID) { m = add_rn(f_m, b_c); p = add_rn(f_c, b_p); }
     else { m = f_m; p = b_p; }
+    return sub_rn(mul_rn(a, m), mul_rn(b, p));
+}
+
+// Column term of the adjoint at one quad from the J slots of the quad (jf, jb) and the three values next to it that the
+// scheme reads: J_F at j0-1 and j0+VEC, J_B at j0+VEC (zero where they are outside the image).
+template <typename T, int VEC, int SCHEME>
+PYTVB_HD void adj_cols(T* out, const T* jf, const T* jb, T jf_left, T jf_right, T jb_right, int j0, int Nj) {
+    T f[VEC + 2], bq[VEC + 2];
+    f[0] = jf_left;
+#pragma unroll
+    for (int e = 0; e < VEC; ++e) f[e + 1] = jf[e];
+    f[VEC + 1] = jf_right;
+#pragma unroll
+    for (int e = 0; e < VEC + 2; ++e) bq[e] = (SCHEME == DOWNWIND) ? f[e] : T(0);
+    if (SCHEME == HYBRID) {
+#pragma unroll
+        for (int e = 0; e < VEC; ++e) bq[e + 1] = jb[e];
+    }
+    if (SCHEME == HYBRID || SCHEME == DOWNWIND) bq[VEC + 1] = jb_right;
+#pragma unroll
+    for (int e = 0; e < VEC; ++e) {
+        T a, b;
+        adj_factors<T, SCHEME>(a, b, j0 + e, Nj, false);
+        out[e] = (SCHEME == CENTRAL) ? adj_term<T, SCHEME>(a, b, f[e], T(0), T(0), f[e + 2], false)
+                                     : adj_term<T, SCHEME>(a, b, f[e], f[e + 1], bq[e + 1], bq[e + 2], false);
+    }
+}
+
+// The in-plane / time prefix of the adjoint, ((rows + t) + cols), and D^T y = (prefix + z) * inv_div: the one order of
+// summation of every path.  (rows + t) alone is what the dual pass stores where a column neighbour lies outside its tile.
+template <typename T, bool T_ON>
+PYTVB_HD T adj_rows_t(T rows, T t) {
+    return T_ON ? add_rn(rows, t) : rows;
+}
+template <typename T, bool T_ON>
+PYTVB_HD T adj_prefix(T rows, T cols, T t) {
+    return add_rn(adj_rows_t<T, T_ON>(rows, t), cols);
+}
+template <typename T, bool Z_ON>
+PYTVB_HD T adj_finish(T prefix, T z, T inv_div) {
+    return mul_rn(Z_ON ? add_rn(prefix, z) : prefix, inv_div);
 }
 
 // Loads of the dual field in the adjoint.  CG = true (generation 3 only, device only): ld.global.cg, because the
@@ -379,9 +473,26 @@ PYTVB_HD T ld_field1(const YT* src) {
     return v;
 }
 
-// D^T y at one quad (times inv_div), strip addressing.
+// Pinned form of scale_by (the time-scale products of the adjoint must round alike wherever they are formed).
+template <typename T, int VEC>
+PYTVB_HD void scale_by_rn(T* v, const T* ts_plane, int o) {
+    if (ts_plane) {
+        const Pack<T, VEC> sc = ld_pack<T, VEC>(ts_plane + o);
+#pragma unroll
+        for (int e = 0; e < VEC; ++e) v[e] = mul_rn(v[e], sc.v[e]);
+    }
+}
+
+// Time term of the adjoint at one quad (before the static factor) from the (time-scaled) slot values; see adj_term.
+template <typename T, int VEC, int SCHEME>
+PYTVB_HD void adj_time(T* out, const T* f_m, const T* f_c, const T* b_c, const T* b_p, const T* fac, T at, T bt, bool fb) {
+#pragma unroll
+    for (int e = 0; e < VEC; ++e) out[e] = mul_rn(adj_term<T, SCHEME>(at, bt, f_m[e], f_c[e], b_c[e], b_p[e], fb), fac[e]);
+}
+
+// In-plane and time prefix of D^T y at one quad (adj_prefix; not yet times inv_div), strip addressing.
 template <typename T, int VEC, int SCHEME, bool Z_ON, bool T_ON, bool CG, typename YT, bool TS>
-PYTVB_HD void strip_quad_DT_impl(T* out, const PrimalPlane<T, YT>& pl, const Params<T>& P, int i, int j0, int o, int o_up, int o_dn) {
+PYTVB_HD void strip_quad_DT_prefix(T* pre, const PrimalPlane<T, YT>& pl, const Params<T>& P, int i, int j0, int o, int o_up, int o_dn) {
     typedef Comp<SCHEME, Z_ON, T_ON> C;
     constexpr bool NF = (SCHEME != DOWNWIND);   // reads the forward-type slot at k-1 (centred: C[k-1])
     constexpr bool NB = (SCHEME != UPWIND);     // reads the backward-type slot at k+1 (centred: C[k+1])
@@ -390,7 +501,7 @@ PYTVB_HD void strip_quad_DT_impl(T* out, const PrimalPlane<T, YT>& pl, const Par
     const YT* yI_B = pl.y + (long long)C::I_B * P.sC;
     const YT* yJ_F = pl.y + (long long)C::J_F * P.sC;
     const YT* yJ_B = pl.y + (long long)C::J_B * P.sC;
-    T acc[VEC];
+    T rows[VEC], cols[VEC], tt[VEC];
     // ---- rows
     {
         T a, b, f_m[VEC], f_c[VEC], b_c[VEC], b_p[VEC];
@@ -400,52 +511,17 @@ PYTVB_HD void strip_quad_DT_impl(T* out, const PrimalPlane<T, YT>& pl, const Par
         if (!CTR && NB) ld_field<T, VEC, CG>(b_c, yI_B + o); else zero_into<T, VEC>(b_c);
         if (NB) ld_field<T, VEC, CG>(b_p, yI_B + o_dn); else zero_into<T, VEC>(b_p);
 #pragma unroll
-        for (int e = 0; e < VEC; ++e) {
-            T m, p;
-            adj_operands<T, SCHEME>(m, p, f_m[e], f_c[e], b_c[e], b_p[e], false);
-            acc[e] = a * m - b * p;
-        }
+        for (int e = 0; e < VEC; ++e) rows[e] = adj_term<T, SCHEME>(a, b, f_m[e], f_c[e], b_c[e], b_p[e], false);
     }
     // ---- columns
     {
-        T f[VEC + 2], bq[VEC + 2];
-#pragma unroll
-        for (int e = 0; e < VEC + 2; ++e) bq[e] = T(0);
-        ld_field<T, VEC, CG>(f + 1, yJ_F + o);
-        f[0] = (NF && j0 > 0) ? ld_field1<T, CG>(yJ_F + o - 1) : T(0);
-        f[VEC + 1] = (CTR && j0 + VEC < P.Nj) ? ld_field1<T, CG>(yJ_F + o + VEC) : T(0);
-        if (SCHEME == HYBRID || SCHEME == DOWNWIND) {
-            if (SCHEME == HYBRID) ld_field<T, VEC, CG>(bq + 1, yJ_B + o);
-            else {
-#pragma unroll
-                for (int e = 0; e < VEC + 2; ++e) bq[e] = f[e];
-            }
-            bq[VEC + 1] = (j0 + VEC < P.Nj) ? ld_field1<T, CG>(yJ_B + o + VEC) : T(0);
-        }
-#pragma unroll
-        for (int e = 0; e < VEC; ++e) {
-            const int j = j0 + e;
-            T a, b, m, p;
-            adj_factors<T, SCHEME>(a, b, j, P.Nj, false);
-            if (CTR) adj_operands<T, SCHEME>(m, p, f[e], T(0), T(0), f[e + 2], false);
-            else adj_operands<T, SCHEME>(m, p, f[e], f[e + 1], bq[e + 1], bq[e + 2], false);
-            acc[e] += a * m - b * p;
-        }
-    }
-    if (Z_ON) {
-        const bool fb = P.z_fwd_fallback != 0;
-        const bool up_form = !CTR || fb;   // needs the slot at k itself
-        T f_m[VEC], f_c[VEC], b_c[VEC], b_p[VEC];
-        if (NF) ld_field<T, VEC, CG>(f_m, pl.zf_m + o); else zero_into<T, VEC>(f_m);
-        if (up_form && NF) ld_field<T, VEC, CG>(f_c, pl.y + (long long)C::Z_F * P.sC + o); else zero_into<T, VEC>(f_c);
-        if (!CTR && NB) ld_field<T, VEC, CG>(b_c, pl.y + (long long)C::Z_B * P.sC + o); else zero_into<T, VEC>(b_c);
-        if (NB && !(CTR && fb)) ld_field<T, VEC, CG>(b_p, pl.zb_p + o); else zero_into<T, VEC>(b_p);
-#pragma unroll
-        for (int e = 0; e < VEC; ++e) {
-            T m, p;
-            adj_operands<T, SCHEME>(m, p, f_m[e], f_c[e], b_c[e], b_p[e], fb);
-            acc[e] += pl.az * m - pl.bz * p;
-        }
+        T jf[VEC], jb[VEC];
+        ld_field<T, VEC, CG>(jf, yJ_F + o);
+        if (SCHEME == HYBRID) ld_field<T, VEC, CG>(jb, yJ_B + o); else zero_into<T, VEC>(jb);
+        const T jf_l = (NF && j0 > 0) ? ld_field1<T, CG>(yJ_F + o - 1) : T(0);
+        const T jf_r = (CTR && j0 + VEC < P.Nj) ? ld_field1<T, CG>(yJ_F + o + VEC) : T(0);
+        const T jb_r = ((SCHEME == HYBRID || SCHEME == DOWNWIND) && j0 + VEC < P.Nj) ? ld_field1<T, CG>(yJ_B + o + VEC) : T(0);
+        adj_cols<T, VEC, SCHEME>(cols, jf, jb, jf_l, jf_r, jb_r, j0, P.Nj);
     }
     if (T_ON) {
         const bool fb = P.t_fwd_fallback != 0;
@@ -456,19 +532,40 @@ PYTVB_HD void strip_quad_DT_impl(T* out, const PrimalPlane<T, YT>& pl, const Par
         if (!CTR && NB) ld_field<T, VEC, CG>(b_c, pl.y + (long long)C::T_B * P.sC + o); else zero_into<T, VEC>(b_c);
         if (NB && !(CTR && fb)) ld_field<T, VEC, CG>(b_p, pl.tb_p + o); else zero_into<T, VEC>(b_p);
         if constexpr (TS) {   // exact adjoint of the per-voxel time scale: every entry is scaled where it lives
-            scale_by<T, VEC>(f_m, pl.ts_m, o); scale_by<T, VEC>(f_c, pl.ts_c, o);
-            scale_by<T, VEC>(b_c, pl.ts_c, o); scale_by<T, VEC>(b_p, pl.ts_p, o);
+            scale_by_rn<T, VEC>(f_m, pl.ts_m, o); scale_by_rn<T, VEC>(f_c, pl.ts_c, o);
+            scale_by_rn<T, VEC>(b_c, pl.ts_c, o); scale_by_rn<T, VEC>(b_p, pl.ts_p, o);
         }
         static_factor<T, VEC>(fac, P, i, j0);
-#pragma unroll
-        for (int e = 0; e < VEC; ++e) {
-            T m, p;
-            adj_operands<T, SCHEME>(m, p, f_m[e], f_c[e], b_c[e], b_p[e], fb);
-            acc[e] += (pl.at * m - pl.bt * p) * fac[e];
-        }
+        adj_time<T, VEC, SCHEME>(tt, f_m, f_c, b_c, b_p, fac, pl.at, pl.bt, fb);
     }
 #pragma unroll
-    for (int e = 0; e < VEC; ++e) out[e] = acc[e] * P.inv_div;
+    for (int e = 0; e < VEC; ++e) pre[e] = adj_prefix<T, T_ON>(rows[e], cols[e], T_ON ? tt[e] : T(0));
+}
+
+// z term of D^T y at one quad (not yet times inv_div).
+template <typename T, int VEC, int SCHEME, bool Z_ON, bool T_ON, bool CG, typename YT>
+PYTVB_HD void strip_quad_DT_z(T* zt, const PrimalPlane<T, YT>& pl, const Params<T>& P, int o) {
+    typedef Comp<SCHEME, Z_ON, T_ON> C;
+    constexpr bool NF = (SCHEME != DOWNWIND), NB = (SCHEME != UPWIND), CTR = (SCHEME == CENTRAL);
+    const bool fb = P.z_fwd_fallback != 0;
+    const bool up_form = !CTR || fb;   // needs the slot at k itself
+    T f_m[VEC], f_c[VEC], b_c[VEC], b_p[VEC];
+    if (NF) ld_field<T, VEC, CG>(f_m, pl.zf_m + o); else zero_into<T, VEC>(f_m);
+    if (up_form && NF) ld_field<T, VEC, CG>(f_c, pl.y + (long long)C::Z_F * P.sC + o); else zero_into<T, VEC>(f_c);
+    if (!CTR && NB) ld_field<T, VEC, CG>(b_c, pl.y + (long long)C::Z_B * P.sC + o); else zero_into<T, VEC>(b_c);
+    if (NB && !(CTR && fb)) ld_field<T, VEC, CG>(b_p, pl.zb_p + o); else zero_into<T, VEC>(b_p);
+#pragma unroll
+    for (int e = 0; e < VEC; ++e) zt[e] = adj_term<T, SCHEME>(pl.az, pl.bz, f_m[e], f_c[e], b_c[e], b_p[e], fb);
+}
+
+// D^T y at one quad (times inv_div), strip addressing.
+template <typename T, int VEC, int SCHEME, bool Z_ON, bool T_ON, bool CG, typename YT, bool TS>
+PYTVB_HD void strip_quad_DT_impl(T* out, const PrimalPlane<T, YT>& pl, const Params<T>& P, int i, int j0, int o, int o_up, int o_dn) {
+    T pre[VEC], zt[VEC];
+    strip_quad_DT_prefix<T, VEC, SCHEME, Z_ON, T_ON, CG, YT, TS>(pre, pl, P, i, j0, o, o_up, o_dn);
+    if (Z_ON) strip_quad_DT_z<T, VEC, SCHEME, Z_ON, T_ON, CG, YT>(zt, pl, P, o); else zero_into<T, VEC>(zt);
+#pragma unroll
+    for (int e = 0; e < VEC; ++e) out[e] = adj_finish<T, Z_ON>(pre[e], zt[e], P.inv_div);
 }
 
 template <typename T, int VEC, int SCHEME, bool Z_ON, bool T_ON, bool CG = false, typename YT = T, bool TS = false>
@@ -476,22 +573,12 @@ PYTVB_HD void strip_quad_DT(T* out, const PrimalPlane<T, YT>& pl, const Params<T
     strip_quad_DT_impl<T, VEC, SCHEME, Z_ON, T_ON, CG, YT, TS && T_ON>(out, pl, P, i, j0, o, o_up, o_dn);
 }
 
-// Primal update at one quad.  VARIANT 0: ROF prox + over-relaxation (aux = xbar); 1: README form (aux = y_f).
-// c1 = 1/(1+tau) (rof) or 1/(1+sigma_A) (readme); c2 = theta or sigma_A.  Returns sum (x_new - x0)^2.
-// `tau` multiplies D^T y: for a normalised half-precision dual the caller passes tau * lam.
-// Other data terms, with v = x - tau D^T y, w = data weight at the voxel (wgt[...] if WM, else 1) and tau_x0 the step of
-// the data term (aux = xbar, c2 = theta, c1 unused):
-//   VARIANT 2: weighted L2, x_new = (v + tau w x0) / (1 + tau w);                  returns sum w (x_new - x0)^2
-//   VARIANT 3: L1,          x_new = x0 + sign(v - x0) max(|v - x0| - tau w, 0);    returns sum w |x_new - x0|
-// (WM is a template parameter for the reason given at strip_raw_diffs_impl.)
-template <typename T, int VEC, int SCHEME, bool Z_ON, bool T_ON, int VARIANT, bool CG = false, typename YT = T, bool TS = false, bool MIR = false,
-          bool WM = false>
-PYTVB_HD T strip_quad_cp_primal(T* x, T* aux, const T* x0, const PrimalPlane<T, YT>& pl, const Params<T>& P, int i, int j0, int o, int o_up, int o_dn,
-                                T tau, T c1, T c2, T tau_x0 = T(-1), MirrorPlanes<T> mir = MirrorPlanes<T>{nullptr, nullptr}, const T* wgt = nullptr) {
-    T dty[VEC];
-    strip_quad_DT<T, VEC, SCHEME, Z_ON, T_ON, CG, YT, TS>(dty, pl, P, i, j0, o, o_up, o_dn);
+// Primal update at one quad given D^T y there (dty); off = offset of the quad in the images.  VARIANT 0: ROF prox + over-relaxation
+// (aux = xbar); 1: README form (aux = y_f).
+template <typename T, int VEC, bool Z_ON, int VARIANT, bool MIR, bool WM>
+PYTVB_HD T cp_primal_update(const T* dty, T* x, T* aux, const T* x0, long long off, int o, T tau, T c1, T c2, T tau_x0, MirrorPlanes<T> mir,
+                            const T* wgt) {
     if (tau_x0 < T(0)) tau_x0 = tau;
-    const long long off = pl.img + o;
     const Pack<T, VEC> xo = ld_pack<T, VEC>(x + off), x0q = ld_pack<T, VEC>(x0 + off);
     Pack<T, VEC> xn, ax;
     T fid = T(0);
@@ -546,6 +633,23 @@ PYTVB_HD T strip_quad_cp_primal(T* x, T* aux, const T* x0, const PrimalPlane<T, 
         if (mir.next) st_pack<T, VEC>(mir.next + o, u);
     }
     return fid;
+}
+
+// The primal update with D^T y read from the dual field, see cp_primal_update.
+// c1 = 1/(1+tau) (rof) or 1/(1+sigma_A) (readme); c2 = theta or sigma_A.  Returns sum (x_new - x0)^2.
+// `tau` multiplies D^T y: for a normalised half-precision dual the caller passes tau * lam.
+// Other data terms, with v = x - tau D^T y, w = data weight at the voxel (wgt[...] if WM, else 1) and tau_x0 the step of
+// the data term (aux = xbar, c2 = theta, c1 unused):
+//   VARIANT 2: weighted L2, x_new = (v + tau w x0) / (1 + tau w);                  returns sum w (x_new - x0)^2
+//   VARIANT 3: L1,          x_new = x0 + sign(v - x0) max(|v - x0| - tau w, 0);    returns sum w |x_new - x0|
+// (WM is a template parameter for the reason given at strip_raw_diffs_impl.)
+template <typename T, int VEC, int SCHEME, bool Z_ON, bool T_ON, int VARIANT, bool CG = false, typename YT = T, bool TS = false, bool MIR = false,
+          bool WM = false>
+PYTVB_HD T strip_quad_cp_primal(T* x, T* aux, const T* x0, const PrimalPlane<T, YT>& pl, const Params<T>& P, int i, int j0, int o, int o_up, int o_dn,
+                                T tau, T c1, T c2, T tau_x0 = T(-1), MirrorPlanes<T> mir = MirrorPlanes<T>{nullptr, nullptr}, const T* wgt = nullptr) {
+    T dty[VEC];
+    strip_quad_DT<T, VEC, SCHEME, Z_ON, T_ON, CG, YT, TS>(dty, pl, P, i, j0, o, o_up, o_dn);
+    return cp_primal_update<T, VEC, Z_ON, VARIANT, MIR, WM>(dty, x, aux, x0, pl.img + o, o, tau, c1, c2, tau_x0, mir, wgt);
 }
 
 // ------------------------------------------------------------------------------------------------
